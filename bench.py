@@ -12,6 +12,8 @@ scaling):
     python bench.py --gpus N --steps K --warmup W            our arm (one process per GPU under torchrun for N > 1)
     python bench.py --impl reference ...                     the CPU arm: the oracle restatement of the reference's
                                                              operators on the host cores, on a bounded sample
+    python bench.py ... --dump-outputs DIR                   also write the last timed step's results to DIR/*.npy, so
+                                                             that two builds can be compared output for output
 
 Prints ONE JSON line (see DESIGN.md "Measurement" for every field).
 """
@@ -282,6 +284,56 @@ def host_keys(table, column_id: int, row_ids: np.ndarray) -> np.ndarray:
     return keys
 
 
+DUMP_SAMPLE_ROWS = 1 << 19   # per RowID output: the five sampled arrays below come to about 32 MB at any scale factor
+DUMP_RUN_ROWS = 1 << 10
+
+
+def dump_positions(total: int) -> np.ndarray:
+    """Positions of a RowID output that --dump-outputs writes: all of them up to DUMP_SAMPLE_ROWS, otherwise runs of
+    DUMP_RUN_ROWS consecutive rows at seeded starts, so the same output length always gives the same positions."""
+    if total <= DUMP_SAMPLE_ROWS:
+        return np.arange(total, dtype=np.int64)
+    starts = np.random.default_rng(0).integers(0, total - DUMP_RUN_ROWS + 1, size=DUMP_SAMPLE_ROWS // DUMP_RUN_ROWS)
+    return np.unique((starts[:, None] + np.arange(DUMP_RUN_ROWS)).ravel())
+
+
+def copy_positions(positions: np.ndarray, copy, sides: int) -> list[np.ndarray]:
+    """RowIDs at `positions`, one device-to-host copy per run of consecutive positions: copy(begin, count, *outputs)."""
+    outputs = [np.empty(len(positions), dtype=ROW_ID_DTYPE) for _ in range(sides)]
+    starts = np.flatnonzero(np.diff(positions, prepend=-2) != 1)
+    for begin, end in zip(starts, np.r_[starts[1:], len(positions)]):
+        copy(int(positions[begin]), int(end - begin), *(output[begin:end].ctypes.data for output in outputs))
+    return outputs
+
+
+def row_id_columns(row_ids: np.ndarray) -> np.ndarray:
+    return np.stack([row_ids["chunk_id"], row_ids["chunk_offset"]], axis=1).astype(np.float64)
+
+
+def dump_outputs(directory: str, prefix: str, device, scan, join, aggregate) -> None:
+    """What the last timed step returned to its caller, as float64 .npy files: the scan's PosList and the join's RowID
+    pairs at the positions of dump_positions (written next to them) with their chunk / radix partition offsets, and the
+    whole Q1 result (group RowIDs, one column per aggregate, NULL flags)."""
+    os.makedirs(directory, exist_ok=True)
+    arrays = {}
+    total, _ = scan.info()
+    positions = dump_positions(total)
+    (rows,) = copy_positions(positions, lambda begin, count, out: capi.check(
+        device.lib.hyb_pos_list_copy(device.ptr, scan.handle, begin, count, out)), 1)
+    arrays.update(scan_positions=positions, scan_row_ids=row_id_columns(rows), scan_chunk_offsets=scan.chunk_offsets())
+    pairs, _, _ = join.info()
+    positions = dump_positions(pairs)
+    build_rows, probe_rows = copy_positions(positions, lambda begin, count, build, probe: capi.check(
+        device.lib.hyb_join_result_copy(device.ptr, join.handle, begin, count, build, probe)), 2)
+    arrays.update(join_positions=positions, join_build_row_ids=row_id_columns(build_rows),
+                  join_probe_row_ids=row_id_columns(probe_rows), join_partition_offsets=join.partition_offsets())
+    arrays.update(aggregate_row_ids=row_id_columns(aggregate.row_ids),
+                  aggregate_values=np.stack([values.astype(np.float64) for values in aggregate.values], axis=1),
+                  aggregate_nulls=np.stack(aggregate.nulls, axis=1))
+    for name, array in arrays.items():
+        np.save(os.path.join(directory, f"{prefix}{name}.npy"), np.asarray(array, dtype=np.float64))
+
+
 def main() -> None:
     parser = argparse.ArgumentParser()
     parser.add_argument("--gpus", type=int, default=1)
@@ -296,7 +348,11 @@ def main() -> None:
     parser.add_argument("--no-verify", action="store_true", help="skip the result self-check (outside the timed region)")
     parser.add_argument("--l2-flush", choices=["auto", "always", "never"], default="auto",
                         help="256 MB memset before every operator: auto = only when an operator input fits the L2")
+    parser.add_argument("--dump-outputs", metavar="DIR",
+                        help="write the results of the last timed step as DIR/<name>.npy (float64; RowID outputs sampled)")
     args = parser.parse_args()
+    if args.steps < 1:
+        parser.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -410,10 +466,13 @@ def main() -> None:
         """hyb_aggregate_hash_distributed: local pre-aggregation, partial groups stored into every peer's arena, merged by all"""
         return group.aggregate_hash(table_l or lineitem, Q1_GROUPBY, Q1_AGGREGATES, Q1_PREDICATES, lineitem_chunk_base, position_base)
 
-    def run_step(record: bool):
+    kept = []
+
+    def run_step(record: bool, keep: bool = False):
         """One step. record=False (warm-up and the TIMED loop): nothing but the operator calls and the reads of their result
         sizes; record=True (a second, untimed loop of the same steps): per-operator CUDA-event statistics are fetched after
-        every call, which synchronises the host with the device and therefore stays out of the timed region."""
+        every call, which synchronises the host with the device and therefore stays out of the timed region. keep=True
+        leaves the step's results alive in `kept` for --dump-outputs instead of freeing them."""
         flush_l2()
         scan = device.table_scan(lineitem, SCAN_PREDICATE)
         scan_stats = device.last_stats() if record else None
@@ -439,8 +498,11 @@ def main() -> None:
                 operators[name].append((stats.dominant_kernel_ms, stats.device_ms, stats.algorithmic_bytes, stats.output_rows))
                 launches[0] += stats.kernel_launches
         result = (scan.info()[0], join.info()[0], aggregate.group_count)
-        scan.free()
-        join.free()
+        if keep:
+            kept[:] = [scan, join, aggregate]
+        else:
+            scan.free()
+            join.free()
         return result
 
     for _ in range(warmup):
@@ -450,11 +512,15 @@ def main() -> None:
     barrier()
     with ClockSampler(local_rank) as clocks:
         begin = time.perf_counter()
-        for _ in range(args.steps):
-            outputs = run_step(False)
+        for step in range(args.steps):
+            outputs = run_step(False, keep=args.dump_outputs is not None and step == args.steps - 1)
         device.synchronize()
         torch.cuda.synchronize()
         elapsed = time.perf_counter() - begin
+    if kept:
+        dump_outputs(args.dump_outputs, "" if world == 1 else f"rank{rank}_", device, *kept)
+        kept[0].free()
+        kept[1].free()
     barrier()
     for _ in range(args.steps):  # the same steps again, instrumented (untimed): per-operator kernel / device times, phases
         run_step(True)

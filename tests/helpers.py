@@ -20,6 +20,10 @@ def tbl(name: str, chunk_size: int = capi.DEFAULT_CHUNK_SIZE) -> Table:
     return load_table(os.path.join(TBL, name), chunk_size)
 
 
+def tpch(name: str):
+    return np.load(os.path.join(TPCH, name))
+
+
 def column_values_at(table: Table, column_id: int, row_ids: np.ndarray):
     """Dereference RowIDs like a ReferenceSegment (reference_segment.hpp): list of python values, None for NULL."""
     out = []

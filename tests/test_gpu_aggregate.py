@@ -5,7 +5,7 @@ import pytest
 
 import oracle_lib as orc
 from aggregate_cases import CASES
-from helpers import ENCODINGS, assert_aggregate_outputs_equal, random_table, tbl
+from helpers import ENCODINGS, assert_aggregate_outputs_equal, random_table, tbl, tpch
 from hyrise_b200 import capi
 from hyrise_b200.device import Aggregate, Expression, Predicate
 from test_oracle_aggregate import (Q1_AGGREGATES, Q1_PREDICATES, Q6_AGGREGATES, Q6_PREDICATES, lineitem_table,
@@ -117,7 +117,7 @@ def test_q1_non_finite_values_stay_in_their_group(device):
     groups. Poisoned rows sit in single groups; the others must still match the oracle to 1e-6."""
     from hyrise_b200.storage import ColumnDefinition, Table
 
-    data = dict(np.load("tests/golden/tpch/sf-0.01_lineitem.npz"))
+    data = dict(tpch("sf-0.01_lineitem.npz"))
     names = ["l_orderkey", "l_quantity", "l_extendedprice", "l_discount", "l_tax", "l_returnflag", "l_linestatus", "l_shipdate"]
     types = [capi.TYPE_INT32] + [capi.TYPE_FLOAT32] * 4 + [capi.TYPE_STRING] * 3
     definitions = [ColumnDefinition(name, data_type) for name, data_type in zip(names, types)]

@@ -3,7 +3,7 @@ import numpy as np
 import pytest
 
 import oracle_lib as orc
-from helpers import ENCODINGS, random_table, row_ids_equal, rows_with_keys, tbl
+from helpers import ENCODINGS, random_table, row_ids_equal, rows_with_keys, tbl, tpch
 from hyrise_b200 import capi
 from hyrise_b200.device import Predicate
 from hyrise_b200.storage import ColumnDefinition, Table
@@ -142,8 +142,8 @@ def test_filtered_inputs(device):
 
 def test_tpch_sf001_orders_lineitem(device):
     # join_hash_test.cpp:26-46 shape on real dbgen data (sf-0.01: 15 000 orders x 60 175 lineitems), reference encodings
-    lineitem = np.load("tests/golden/tpch/sf-0.01_lineitem.npz")
-    orders = np.load("tests/golden/tpch/sf-0.01_orders.npz")
+    lineitem = tpch("sf-0.01_lineitem.npz")
+    orders = tpch("sf-0.01_orders.npz")
     orders_table = Table.from_columns([ColumnDefinition("o_orderkey", capi.TYPE_INT32)], [orders["o_orderkey"]],
                                       chunk_size=4_000).encode("Unencoded")
     lineitem_table = Table.from_columns([ColumnDefinition("l_orderkey", capi.TYPE_INT32)], [lineitem["l_orderkey"]],

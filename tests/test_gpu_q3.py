@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 
 import oracle_lib as orc
-from helpers import row_ids_equal
+from helpers import row_ids_equal, tpch
 from hyrise_b200 import capi
 from hyrise_b200.device import Aggregate, Expression, Predicate
 from hyrise_b200.storage import ColumnDefinition, Table
@@ -23,7 +23,7 @@ Q3_SQL = """SELECT l_orderkey, SUM(l_extendedprice*(1.0-l_discount)) as revenue,
 
 
 def load(name, columns, chunk_size, encoding="Automatic"):
-    data = np.load(f"tests/golden/tpch/sf-0.01_{name}.npz")
+    data = tpch(f"sf-0.01_{name}.npz")
     definitions, arrays = [], []
     for column in columns:
         values = data[column]

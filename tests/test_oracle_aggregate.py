@@ -8,7 +8,7 @@ import pytest
 
 import oracle_lib as orc
 from aggregate_cases import CASES
-from helpers import aggregate_rows, assert_rows_match_unordered, expected_rows, tbl
+from helpers import aggregate_rows, assert_rows_match_unordered, expected_rows, tbl, tpch
 from hyrise_b200 import capi
 from hyrise_b200.device import Aggregate, Expression, Predicate
 from hyrise_b200.storage import ColumnDefinition, Table
@@ -69,7 +69,7 @@ def test_group_order_and_immediate_keys():
 
 
 def lineitem_table(scale="sf-0.01", chunk_size=10_000):
-    data = np.load(f"tests/golden/tpch/{scale}_lineitem.npz")
+    data = tpch(f"{scale}_lineitem.npz")
     names = ["l_orderkey", "l_quantity", "l_extendedprice", "l_discount", "l_tax", "l_returnflag", "l_linestatus", "l_shipdate"]
     types = [capi.TYPE_INT32] + [capi.TYPE_FLOAT32] * 4 + [capi.TYPE_STRING] * 3
     definitions = [ColumnDefinition(name, data_type) for name, data_type in zip(names, types)]

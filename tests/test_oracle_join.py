@@ -6,7 +6,7 @@ import numpy as np
 import pytest
 
 import oracle_lib as orc
-from helpers import join_result_rows, rows_with_keys, tbl, verification_join
+from helpers import join_result_rows, rows_with_keys, tbl, tpch, verification_join
 from hyrise_b200 import capi
 from hyrise_b200.storage import ColumnDefinition, Table
 
@@ -92,8 +92,8 @@ def test_join_test_runner_inputs(mode, radix_bits, sizes, chunk_size):
 
 def test_tpch_sf0001_join():
     # join_hash_test.cpp:26-46, 70-82: orders x lineitem on orderkey, chunk size 10, 10 radix bits -> use the maximum 8
-    lineitem = np.load("tests/golden/tpch/sf-0.001_lineitem.npz")
-    orders = np.load("tests/golden/tpch/sf-0.001_orders.npz")
+    lineitem = tpch("sf-0.001_lineitem.npz")
+    orders = tpch("sf-0.001_orders.npz")
     orders_table = Table.from_columns([ColumnDefinition("o_orderkey", capi.TYPE_INT32)], [orders["o_orderkey"]],
                                       chunk_size=10)
     lineitem_table = Table.from_columns([ColumnDefinition("l_orderkey", capi.TYPE_INT32)], [lineitem["l_orderkey"]],
